@@ -19,6 +19,10 @@ The CPU legs (`cpu_baseline` of the default run, `--impl reference`) run the UNM
 /root/reference into git-ignored baseline/_ref by __graft_entry__.build() (kind "reference"); only if that package is
 absent they fall back to oracle/torch_port.py (kind "port").  The measured arm imports neither: it builds its learners
 and synthetic data from `rl_replicas_b200.synthetic` alone.
+
+  --dump-outputs DIR : after the timed steps, write what the last step of each timed leg computed as DIR/<name>.npy
+                       (parameters, Adam moments and update statistics; inputs are seeded, so two builds can be compared
+                       output for output).
 """
 from __future__ import annotations
 
@@ -74,6 +78,47 @@ def make_batch(n_envs, horizon, pl, seed):
         return h
 
     return synthetic.fixed_batch(n_envs, horizon, OBS, ACT, seed=seed, frac_not_done=0.1, mean_fn=mean_fn)
+
+
+# UpdateStats fields that are results of the update (kernel_launches / fused describe how it ran, not what it computed)
+STAT_FIELDS = ("policy_loss_before", "entropy_before", "logp_std_before", "kl_divergence", "value_loss_mean",
+               "policy_steps_applied", "value_steps_applied", "adv_mean", "adv_std", "value_loss_first", "value_loss_last")
+
+
+def stats_array(stats):
+    return np.array([float(getattr(stats, f)) for f in STAT_FIELDS], dtype=np.float64)
+
+
+def learner_outputs(prefix, ppo):
+    """What PPO.train leaves its caller: the networks' parameters, the Adam moments and step, the update statistics."""
+    from rl_replicas_b200.algorithms._onpolicy import describe_mlp, flat_params, read_adam_state
+    out = {f"{prefix}_stats": stats_array(ppo.last_update_stats)}
+    for name, module in (("policy", ppo.policy), ("value", ppo.value_function)):
+        linears = describe_mlp(module.network)[3]
+        m, v, step = read_adam_state(module.optimizer, linears)
+        out.update({f"{prefix}_{name}_params": flat_params(linears), f"{prefix}_{name}_adam_exp_avg": m,
+                    f"{prefix}_{name}_adam_exp_avg_sq": v, f"{prefix}_{name}_adam_step": np.float64(step)})
+    return out
+
+
+def engine_outputs(prefix, engine, stats):
+    """What OnPolicyEngine.update leaves its caller: the returned statistics and the device-resident parameters and
+    Adam state, read back."""
+    from rl_replicas_b200.engine import POLICY, VALUE
+    out = {f"{prefix}_stats": stats_array(stats)}
+    for name, which in (("policy", POLICY), ("value", VALUE)):
+        m, v, step = engine.get_adam(which)
+        out.update({f"{prefix}_{name}_params": engine.get_params(which), f"{prefix}_{name}_adam_exp_avg": m,
+                    f"{prefix}_{name}_adam_exp_avg_sq": v, f"{prefix}_{name}_adam_step": np.float64(step)})
+    return out
+
+
+def dump_outputs(directory, arrays):
+    """DIR/<name>.npy per array, as float32 or float64."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(directory, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -248,8 +293,14 @@ def main():
     ap.add_argument("--horizon", type=int, default=1000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the TRPO (config 3) / TD3 (config 4) side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each PPO leg computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU arm")
         return run_reference_arm(args)
 
     import torch
@@ -328,15 +379,20 @@ def main():
     ms_e2e = timed(lambda: ppo.train(store), args.steps, args.warmup)  # the reference's boundary call (ppo.py:139)
     fused_path = int(ppo.last_update_stats.fused)
     launches_per_step = (lib.b200rl_launch_count() - l0) // (args.steps + args.warmup)
+    dump = bool(args.dump_outputs) and rank == 0
+    outputs = learner_outputs("e2e", ppo) if dump else {}
 
     # ---------------- value: batch resident in HBM ----------------
     engine = ppo._engine
     hp = ppo._hparams(engine, n_local * world if distributed else 0)
+    last = {}
 
     def device_step():
-        engine.update(hp, "ppo", None, distributed)
+        last["stats"] = engine.update(hp, "ppo", None, distributed)
 
     ms_dev = timed(device_step, args.steps, args.warmup)
+    if dump:  # read back before the per-stage timings below move the engine's state on
+        outputs.update(engine_outputs("update", engine, last["stats"]))
     clocks = sampler.summary() if sampler else None
 
     # ---------------- kernel-level rooflines (rank 0, N = 1 semantics: per-GPU kernels) ----------------
@@ -599,6 +655,8 @@ def main():
         if not args.no_cpu_baseline and world == 1:
             cb, _ = cpu_reference_run(2, 1)
             line["cpu_baseline"] = cb
+        if dump:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if distributed:
         dist.destroy_process_group()

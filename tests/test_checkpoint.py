@@ -1,12 +1,9 @@
 """Checkpoint parity + resume (SURVEY 8f-3): save_model writes the reference's dictionary layout, load_model restores
-networks, Adam state and step counters; checkpoints shipped with the reference load as warm starts (build container
-only: skipped where /root/reference is absent)."""
-import glob
+networks, Adam state and step counters; checkpoints written the way the reference writes them load as warm starts."""
 import os
 import types
 
 import numpy as np
-import pytest
 import torch
 
 
@@ -98,18 +95,80 @@ def test_td3_checkpoint_round_trip(tmp_path):
     assert not any(p.requires_grad for p in b.target_policy.network.parameters())
 
 
-REF_CKPTS = sorted(glob.glob("/root/reference/benchmarks/*/*/seed-0/model.pt"))
+class _ReferenceMLP(torch.nn.Module):
+    """The reference's network layout (ref networks/mlp.py): Linear / activation pairs in ``self.network``, so the
+    state-dict keys read network.<i>.weight / network.<i>.bias."""
+
+    def __init__(self, sizes, activation, output_activation=torch.nn.Identity):
+        super().__init__()
+        layers = []
+        for i in range(len(sizes) - 1):
+            layers += [torch.nn.Linear(sizes[i], sizes[i + 1]),
+                       activation() if i < len(sizes) - 2 else output_activation()]
+        self.network = torch.nn.Sequential(*layers)
+
+    def forward(self, x):
+        return self.network(x)
 
 
-@pytest.mark.skipif(not REF_CKPTS, reason="reference checkpoints are only present in the build container")
-def test_reference_shipped_checkpoints_load_as_warm_starts():
-    """One checkpoint per algorithm family found: layer sizes come from the file, the loaded module reproduces a
-    plain-torch evaluation of the stored weights."""
+# Adam's param-group keys in torch 2.5.1, the version the reference pins (pyproject.toml): newer torch adds others
+_ADAM_GROUP_KEYS_TORCH_2_5 = {"params", "lr", "betas", "eps", "weight_decay", "amsgrad", "maximize", "foreach",
+                              "capturable", "differentiable", "fused"}
+
+
+def _trained(sizes, activation, output_activation=torch.nn.Identity):
+    """A network and its Adam state dict after a few real steps (moments and a step count), laid out as torch 2.5.1
+    writes it."""
+    net = _ReferenceMLP(sizes, activation, output_activation)
+    opt = torch.optim.Adam(net.parameters(), lr=1e-3)
+    for _ in range(3):
+        opt.zero_grad()
+        net(torch.randn(8, sizes[0])).pow(2).mean().backward()
+        opt.step()
+    sd = opt.state_dict()
+    sd["param_groups"] = [{k: v for k, v in g.items() if k in _ADAM_GROUP_KEYS_TORCH_2_5} for g in sd["param_groups"]]
+    return net, sd
+
+
+def _reference_checkpoints(directory):
+    """{algorithm: path} of checkpoints with the dictionaries the reference's save_model writes (ref ppo.py:296-306;
+    vpg.py and trpo.py use the same keys; td3.py:367-382), built from plain torch modules at the shapes of the shipped
+    benchmark checkpoints: HalfCheetah [64, 32] nets (17 -> 64 -> 32 -> 6 policy, 17 -> 64 -> 32 -> 1 value, tanh;
+    run_ppo.py:28-29), used here for PPO, VPG and TRPO, and TD3 on Hopper (11 -> 256 -> 256 -> 3 policy, relu with tanh
+    output; 14 -> 256 -> 256 -> 1 critics).  TRPO's
+    policy optimizer is the conjugate-gradient one, whose state dict holds its hyper-parameters and no per-parameter
+    state (ref optimizers/conjugate_gradient_optimizer.py:100-119)."""
+    torch.manual_seed(0)
+    paths = {}
+    for epoch, algo in enumerate(("ppo", "vpg", "trpo"), start=1):
+        (pnet, popt), (vnet, vopt) = _trained([17, 64, 32, 6], torch.nn.Tanh), _trained([17, 64, 32, 1], torch.nn.Tanh)
+        if algo == "trpo":
+            popt = {"state": {"max_constraint": 0.01, "n_conjugate_gradients": 10, "max_backtracks": 15,
+                              "backtrack_ratio": 0.8, "hvp_damping_coefficient": 1e-5},
+                    "param_groups": [{"params": list(range(6))}]}
+        paths[algo] = os.path.join(directory, algo + ".pt")
+        torch.save({"epoch": 100 * epoch, "total_steps": 400000 * epoch,
+                    "policy_state_dict": pnet.state_dict(), "policy_optimizer_state_dict": popt,
+                    "value_function_state_dict": vnet.state_dict(), "value_function_optimizer_state_dict": vopt},
+                   paths[algo])
+    pnet, popt = _trained([11, 256, 256, 3], torch.nn.ReLU, torch.nn.Tanh)
+    ckpt = {"epoch": 300, "total_steps": 1000000,
+            "policy_state_dict": pnet.state_dict(), "policy_optimizer_state_dict": popt,
+            "target_policy_state_dict": _ReferenceMLP([11, 256, 256, 3], torch.nn.ReLU, torch.nn.Tanh).state_dict()}
+    for q in ("q_function_1", "q_function_2"):
+        qnet, qopt = _trained([14, 256, 256, 1], torch.nn.ReLU)
+        ckpt.update({f"{q}_state_dict": qnet.state_dict(), f"{q}_optimizer_state_dict": qopt,
+                     f"target_{q}_state_dict": _ReferenceMLP([14, 256, 256, 1], torch.nn.ReLU).state_dict()})
+    paths["td3"] = os.path.join(directory, "td3.pt")
+    torch.save(ckpt, paths["td3"])
+    return paths
+
+
+def test_reference_layout_checkpoints_load_as_warm_starts(tmp_path):
+    """One checkpoint per algorithm family: layer sizes come from the file, the loaded module reproduces a plain-torch
+    evaluation of the stored weights."""
     seen = set()
-    for path in REF_CKPTS:
-        algo_name = path.split("/")[-3]
-        if algo_name in seen:
-            continue
+    for algo_name, path in _reference_checkpoints(str(tmp_path)).items():
         seen.add(algo_name)
         ckpt = torch.load(path, map_location="cpu", weights_only=False)
         sd = ckpt["policy_state_dict"]
@@ -139,4 +198,4 @@ def test_reference_shipped_checkpoints_load_as_warm_starts():
         else:
             continue
         assert epoch == ckpt["epoch"] and algo.current_total_steps == ckpt["total_steps"]
-    assert seen
+    assert seen == {"ppo", "vpg", "trpo", "td3"}
