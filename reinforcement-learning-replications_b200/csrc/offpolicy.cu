@@ -223,10 +223,11 @@ __global__ void gather_rows_kernel(const float* table, const long long* idx, int
   out[i] = table[idx[r] * width + (i - r * width)];
 }
 
-// y = r + gamma * (1 - d) * min(q1t, q2t)   (td3.py:337-339; ddpg.py:280: single target Q)
+// y = r + gamma * (1 - d) * min(q1t, q2t)   (td3.py:337-339; ddpg.py:280: single target Q).  Every product and the sum
+// rounded on its own, as the reference's float32 tensor ops do: written plainly, nvcc fuses the last two into an FFMA.
 __device__ __forceinline__ float td_target(float rew, float done, float q1t, const float* q2t, int i, float gamma) {
   const float q = q2t ? fminf(q1t, q2t[i]) : q1t;
-  return rew + gamma * (1.f - done) * q;
+  return __fadd_rn(rew, __fmul_rn(__fmul_rn(gamma, 1.f - done), q));
 }
 
 // One CTA: the critic's loss with its TD target computed on the fly: y as above, loss = mean((q - y)^2),
@@ -260,7 +261,11 @@ __global__ void __launch_bounds__(GTHREADS) q_loss_kernel(const float* q, const 
   }
 }
 
-// target <- rho * target + (1 - rho) * param   (utils.py:47-57: f32 tensors tensor(rho), tensor(1 - rho))
+// target <- rho * target + (1 - rho) * param   (utils.py:47-57: f32 tensors tensor(rho), tensor(1 - rho)): two rounded
+// products and a rounded sum, never an FFMA (the same rule as b200rl_polyak in utils_kernels.cu)
+__device__ __forceinline__ float polyak(float rho, float target, float one_minus_rho, float param) {
+  return __fadd_rn(__fmul_rn(rho, target), __fmul_rn(one_minus_rho, param));
+}
 struct PolyakArgs {
   float* target[3];
   const float* param[3];
@@ -270,7 +275,7 @@ struct PolyakArgs {
 __global__ void polyak_kernel(const PolyakArgs a, float rho, float one_minus_rho) {  // every network in one launch
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   for (int k = 0; k < a.n_nets; ++k)
-    if (i < a.n[k]) a.target[k][i] = rho * a.target[k][i] + one_minus_rho * a.param[k][i];
+    if (i < a.n[k]) a.target[k][i] = polyak(rho, a.target[k][i], one_minus_rho, a.param[k][i]);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -398,7 +403,7 @@ __global__ void __launch_bounds__(GTHREADS, 2) offpolicy_mega_kernel(const MkBlo
         }
       } else if (type == MK_POLYAK) {
         const int i = local * GTHREADS + threadIdx.x;
-        if (i < op.n) op.o0[i] = op.f0 * op.o0[i] + op.f1 * op.p0[i];
+        if (i < op.n) op.o0[i] = polyak(op.f0, op.o0[i], op.f1, op.p0[i]);
       } else {  // MK_FILL
         const int i = local * GTHREADS + threadIdx.x;
         if (i < op.n) op.o0[i] = op.f0;
